@@ -12,7 +12,7 @@ default run to last > 0.5 s.
   latency   B = 1: one stereo frame per step (graph replay, device-resident; and end to end through orbr_*), p50 / p99
   parity    the first frames of the run against the CPU oracle, before anything is timed (the run aborts on a mismatch)
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3|5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3|5] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); frames shard across ranks with no data-path collective (weak scaling).  The
 `config5` section (1280x720 stereo, 2000 features, one sequence per rank) adds the one exchange the design has: the NCCL
@@ -696,6 +696,49 @@ class Workload:
         return {"ok": True, "against": "CPU oracle (oracle/), same images and query sets, through orbr_submit / orbr_collect", **checked,
                 "compared": "keypoint records (28 B), descriptors, mvuRight / mvDepth float bits, both match arrays: identical"}
 
+    def dump_batch(self, i, out_dir, budget=64 << 20):
+        """Writes what batch i returned to its caller as out_dir/<name>.npy, read back from the handle that ran it -- valid until that
+        handle runs another batch.  Stereo pairs p = 0, 1, ... are kept while the files fit in `budget` bytes.  All float32 but
+        image_offsets (float64); integers are exact in both.
+          keypoints (rows, 7)         x, y, size, angle, response, octave, class_id of every keypoint, images L0 R0 L1 R1 ...
+          image_offsets (2P + 1)      first row of each image in keypoints / descriptors
+          descriptors (rows, 32)      descriptor bytes, one row per keypoint
+          uright_left, depth_left     mvuRight / mvDepth, one per LEFT-image keypoint (left images' rows in pair order; -1: none)
+          last_frame_match_left       one per left-image keypoint: the matched query of SearchByProjection(cur, last), as an index
+                                      into the batch's whole last-frame query list (pair p's queries follow pair p-1's); -1: none
+          local_map_match             one per local-map query (the batch's list, pairs in order): the matched keypoint of
+                                      SearchByProjection(F, local points), as an index into that pair's left image; -1: none
+          matches_per_frame (P, 2)    matches of the last-frame and of the local-map search per stereo pair"""
+        self.torch.cuda.synchronize()
+        k, pb, B = i % self.NH, i % self.pool_batches, self.B
+        e = self.exs[k]
+        _, _, off, kps, desc = e.download(self.nimg)
+        uR, dep = e.stereo_download(int(off[-1]))
+        fm, nm, mt = self.d_fm[k].cpu().numpy(), self.d_nm[k].cpu().numpy(), self.d_match[k].cpu().numpy()
+        loff = self.H_LOC[pb]["off"]
+        n_pairs, used = 0, 0
+        while n_pairs < B:
+            rows, left = int(off[2 * n_pairs + 2] - off[2 * n_pairs]), int(off[2 * n_pairs + 1] - off[2 * n_pairs])
+            need = rows * (7 + 32) * 4 + left * 3 * 4 + int(loff[n_pairs + 1] - loff[n_pairs]) * 4 + 2 * 4 + 2 * 8
+            if used + need > budget - (1 << 16):
+                break
+            used += need
+            n_pairs += 1
+        if n_pairs == 0:
+            raise SystemExit(f"--dump-outputs: one stereo pair of batch {i} does not fit in {budget} bytes")
+        rows, left = int(off[2 * n_pairs]), np.concatenate([np.arange(off[2 * p], off[2 * p + 1]) for p in range(n_pairs)]).astype(np.int64)
+        kp = kps[:rows]
+        out = {"keypoints": np.stack([kp["x"], kp["y"], kp["size"], kp["angle"], kp["response"], kp["octave"], kp["class_id"]], 1).astype(np.float32),
+               "image_offsets": off[:2 * n_pairs + 1].astype(np.float64), "descriptors": desc[:rows].astype(np.float32),
+               "uright_left": uR[left].astype(np.float32), "depth_left": dep[left].astype(np.float32),
+               "last_frame_match_left": fm[left].astype(np.float32), "local_map_match": mt[:int(loff[n_pairs])].astype(np.float32),
+               "matches_per_frame": np.stack([nm[:n_pairs], nm[B:B + n_pairs]], 1).astype(np.float32)}
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in out.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+        return {"dir": out_dir, "batch": i, "stereo_pairs": n_pairs, "of": B, "bytes": int(sum(a.nbytes for a in out.values())),
+                "sample": "the last batch of the last timed step (one of --batches-per-step batches), first stereo_pairs pairs"}
+
     def close(self):
         for (k, _, _), g in self.graphs.items():
             self.exs[k].graph_destroy(g)
@@ -862,7 +905,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of CUDA-graph replays in the value leg")
     ap.add_argument("--e2e-repeats", type=int, default=5)
     ap.add_argument("--latency-frames", type=int, default=200)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last batch of the last step returned (a "
+                    "one-batch sample of the step: keypoints, descriptors, mvuRight, mvDepth, both match arrays) as DIR/<name>.npy, "
+                    "to compare two builds on the same seeded inputs (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -921,6 +971,7 @@ def main():
     ms_max = max_ranks(ms)
     value = world * B * BPS * args.steps / (ms_max * 1e-3)
     nm_host = wl.d_nm[0].cpu().numpy()
+    dumped = wl.dump_batch(nwarm + args.steps * BPS - 1, args.dump_outputs) if args.dump_outputs and rank == 0 else None
     kernels_per_batch = wl.exs[0].graph_kernels(wl.graphs[(0, 0, False)]) if use_graph else launches // (args.steps * BPS)
 
     # ---- per-stage times for the roofline: a serial (un-overlapped, eager) pass over the same batches, CUDA events per stage ----
@@ -1099,7 +1150,7 @@ def main():
                         "repeats_frames_per_s": e2e_rates, "spread": (max(e2e_rates) - min(e2e_rates)) / e2e_value if e2e_value else None,
                         "api": "orbr_submit / orbr_collect (pinned host buffers in and out), one host thread, median of the repeats"},
                 "gpu_launches": int(launches), "graph_launches": int(args.steps * BPS) if use_graph else 0, "kernels_per_batch": int(kernels_per_batch),
-                "clocks": clocks, "parity": parity, "roofline": roofline, "cpu_baseline": cpu, "latency_b1": latency, "chained_flow": chained, "config5": cfg5, **side}
+                "clocks": clocks, "parity": parity, "dumped_outputs": dumped, "roofline": roofline, "cpu_baseline": cpu, "latency_b1": latency, "chained_flow": chained, "config5": cfg5, **side}
         print(json.dumps(line))
     wl.close()
     if world > 1:

@@ -12,9 +12,10 @@ sys.path.insert(0, ROOT)
 import bench  # noqa: E402
 from oracle import pyoracle as po  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not bench.reference_source_available(), reason="oracle/_ref is not built and /root/reference is absent")
+needs_ref = pytest.mark.skipif(not bench.reference_source_available(), reason="oracle/_ref is not built and no reference checkout is given")
 
 
+@needs_ref
 def test_reference_source_frame_equals_the_oracle_frame():
     c = bench.CONFIGS[3]
     pairs = bench.make_pairs(2, c["W"], c["H"], base=4)
@@ -26,6 +27,7 @@ def test_reference_source_frame_equals_the_oracle_frame():
         assert n == int((o["fm"] >= 0).sum()) + int((o["mt"] >= 0).sum()) and n > 1000
 
 
+@needs_ref
 def test_threaded_drivers_run():
     c = bench.CONFIGS[3]
     pairs = bench.make_pairs(4, c["W"], c["H"], base=4)
